@@ -326,6 +326,25 @@ def record_tokens(unet, text):
     return seen, hooks
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, trainer, loss):
+    """What the timed step hands its caller after the last timed step, as float32 .npy files: the
+    loss and every trained LoRA factor (the fp32 masters the model's Parameters view, unet sites
+    then text encoder, up before down). Above DUMP_LIMIT_BYTES the factors are a fixed seeded sample."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    p = trainer.arena.p.detach().cpu()
+    factors = torch.cat([p[o:o + n] for _, _, _, o, n in trainer.arena.entries])
+    limit = (DUMP_LIMIT_BYTES - 4096) // 4          # room for the .npy headers and loss.npy
+    if factors.numel() > limit:
+        idx = torch.randperm(factors.numel(), generator=torch.Generator().manual_seed(0))[:limit]
+        factors = factors[idx.sort().values]
+    np.save(os.path.join(out_dir, "loss.npy"), np.asarray([loss], dtype=np.float32))
+    np.save(os.path.join(out_dir, "lora_factors.npy"), factors.numpy().astype(np.float32))
+
+
 def run_native(args):
     import torch.distributed as dist
     from lora_b200 import ops
@@ -456,6 +475,8 @@ def run_native(args):
     barrier()
     ms_e2e = e2.elapsed_time(e3)
     loss_e2e = float(hl.item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, trainer, loss_e2e)
 
     t = torch.tensor([ms_dev, ms_e2e], device=dev, dtype=torch.float64)
     if world > 1:
@@ -725,6 +746,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-cuda-baseline", action="store_true", help="skip the reference-on-this-GPU block")
     ap.add_argument("--cpu-budget", type=float, default=25.0, help="seconds of CPU-baseline work")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's loss and LoRA factors as DIR/<name>.npy")
     args = ap.parse_args()
     out = (run_reference(args) if args.impl == "reference" else
            run_reference_cuda(args) if args.impl == "reference-cuda" else run_native(args))

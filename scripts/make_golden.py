@@ -17,6 +17,11 @@ Outputs (all small, committed):
   golden/pti_loss_step.pt               cli_lora_pti.loss_step losses (plain / t_mult / masked / inpainting)
   golden/ti_train_inversion.pt          cli_lora_pti.train_inversion: 3 real steps (grads, lr, rows after)
   golden/pti_perform_tuning.pt          cli_lora_pti.perform_tuning: 3 real steps (losses, lrs, all factors after)
+  golden/reference_live.json            namespace, signatures and tiny-model outputs of lora.py (digests)
+  golden/reference_modules_fp32.pt      the operator classes' fp32 forward + backward on small inputs
+  golden/reference_formats.json         lora_join, cli_lora_add.add, to_ckpt_v2 key conversion (digests)
+
+    python scripts/make_golden.py live formats        (only the named generators)
 """
 import hashlib
 import importlib.util
@@ -464,16 +469,244 @@ def gen_tuning(R):
     print("tuning", [(r["loss"], r["lrs"]) for r in rec], len(sites))
 
 
+def _sites(model):
+    return [m for m in model.modules() if type(m).__name__.startswith("LoraInjected")]
+
+
+def _load_ref(fname, modname):
+    """Load one reference file as a sub-module of a stub package `lora_diffusion_ref` whose `.lora` is
+    the real lora.py; `fire` and `diffusers` are empty stand-ins (only imported, never called here)."""
+    stubs = {"fire": {"Fire": lambda *a, **k: None}, "diffusers": {"StableDiffusionPipeline": object}}
+    planted = []
+    for stub, attrs in stubs.items():
+        if stub not in sys.modules:
+            m = types.ModuleType(stub)
+            for k, v in attrs.items():
+                setattr(m, k, v)
+            sys.modules[stub] = m
+            planted.append(stub)
+    try:
+        if "lora_diffusion_ref" not in sys.modules:
+            pkg = types.ModuleType("lora_diffusion_ref")
+            pkg.__path__ = [f"{REF}/lora_diffusion"]
+            sys.modules["lora_diffusion_ref"] = pkg
+        full = f"lora_diffusion_ref.{modname}"
+        if full in sys.modules:
+            return sys.modules[full]
+        spec = importlib.util.spec_from_file_location(full, f"{REF}/lora_diffusion/{fname}")
+        mod = importlib.util.module_from_spec(spec)
+        sys.modules[full] = mod
+        spec.loader.exec_module(mod)
+    finally:
+        for stub in planted:
+            sys.modules.pop(stub, None)
+    return mod
+
+
+def gen_live(R):
+    """tests/test_vs_reference_live.py: the reference's public namespace and signatures, and its
+    outputs on the tiny host models for the same seeded calls the tests make with lora_b200 (each
+    side is also checked against lora_b200 here). Tensors as digests (tests/refgold.py), except the
+    fp32 operator case, which is stored whole because it is compared with a tolerance."""
+    import copy
+    import inspect
+    import tempfile
+    import warnings
+    from safetensors import safe_open
+    import lora_b200 as L
+    from lora_b200.host.clip import build_text_encoder
+    from lora_b200.host.unet_sd15 import UNet2DConditionModel, UNetConfig
+    from refgold import canon_metadata, canon_signature, digest
+    out = {}
+    tmp = tempfile.mkdtemp()
+
+    # ---- namespace and signatures
+    names = {n for n in dir(R) if not n.startswith("_") and (callable(getattr(R, n)) or n.isupper()
+             or n in ("safetensors_available",))}
+    skip = {"Callable", "Dict", "List", "Optional", "Set", "Tuple", "Type", "Union", "groupby", "F", "nn",
+            "np", "PIL", "torch", "json", "math", "_find_modules_old"}
+    out["namespace"] = sorted(n for n in names if n not in skip and not inspect.ismodule(getattr(R, n)))
+    signed = ["inject_trainable_lora", "inject_trainable_lora_extended", "monkeypatch_or_replace_lora",
+              "monkeypatch_or_replace_lora_extended", "patch_pipe", "save_all", "tune_lora_scale",
+              "monkeypatch_add_lora", "apply_learned_embed_in_clip", "extract_lora_as_tensor",
+              "LoraInjectedLinear.__init__", "LoraInjectedConv2d.__init__"]
+    out["signatures"] = {}
+    for n in signed:
+        obj = R
+        for part in n.split("."):
+            obj = getattr(obj, part)
+        out["signatures"][n] = canon_signature(obj)
+
+    # ---- inject (extended unet + text encoder), save_all, load the file back, collapse
+    torch.manual_seed(0)
+    unet, te = UNet2DConditionModel(UNetConfig.tiny()), build_text_encoder(tiny=True)
+    torch.manual_seed(1)
+    _, n2 = R.inject_trainable_lora_extended(unet, r=4)
+    _, t2 = R.inject_trainable_lora(te, target_replace_module={"CLIPAttention"}, r=4)
+    refs = _sites(unet) + _sites(te)
+    rec = {"unet_names": n2, "text_names": t2, "kinds": [type(m).__name__ for m in refs],
+           "down": [digest(m.lora_down.weight) for m in refs]}
+    g = torch.Generator().manual_seed(2)
+    for m in refs:
+        m.lora_up.weight.data.normal_(0, 0.05, generator=g)
+    R.tune_lora_scale(unet, 0.7)
+    path = os.path.join(tmp, "b.safetensors")
+    R.save_all(unet, te, path, save_ti=False, target_replace_module_unet=R.UNET_EXTENDED_TARGET_REPLACE)
+    f = safe_open(path, "pt")
+    rec["saved"] = {k: digest(f.get_tensor(k)) for k in f.keys()}
+    rec["saved_metadata"] = canon_metadata(f.metadata())
+
+    class P:
+        pass
+    pr = P()
+    torch.manual_seed(0)
+    pr.unet, pr.text_encoder = UNet2DConditionModel(UNetConfig.tiny()), build_text_encoder(tiny=True)
+    R.monkeypatch_or_replace_safeloras(pr, f)
+    rec["loaded"] = [[type(m).__name__, digest(m.lora_up.weight), digest(m.lora_down.weight)]
+                     for m in _sites(pr.unet) + _sites(pr.text_encoder)]
+    R.collapse_lora(pr.unet, 0.5)
+    rec["collapsed"] = [digest(m.linear.weight if hasattr(m, "linear") else m.conv.weight) for m in _sites(pr.unet)]
+    out["inject_save_load"] = rec
+
+    # ---- the reference operator classes, fp32, fwd + bwd (stored whole: compared with a tolerance)
+    torch.manual_seed(3)
+    ops = []
+    for conv in (False, True):
+        if conv:
+            base = nn.Conv2d(8, 12, 3, padding=1)
+            ref = R.LoraInjectedConv2d(8, 12, 3, 1, 1, r=4, dropout_p=0.0, scale=1.3)
+            ref.conv.weight, ref.conv.bias = base.weight, base.bias
+            x = torch.randn(2, 8, 7, 7)
+        else:
+            base = nn.Linear(24, 40)
+            ref = R.LoraInjectedLinear(24, 40, True, r=4, dropout_p=0.0, scale=1.3)
+            ref.linear.weight, ref.linear.bias = base.weight, base.bias
+            x = torch.randn(3, 5, 24)
+        ref.lora_up.weight.data.normal_(0, 0.1)
+        x1 = x.clone().requires_grad_(True)
+        y = ref(x1)
+        gy = torch.randn_like(y)
+        y.backward(gy)
+        ops.append({k: v.detach().clone() for k, v in dict(
+            W=base.weight, b=base.bias, down=ref.lora_down.weight, up=ref.lora_up.weight, x=x, gy=gy, y=y,
+            dX=x1.grad, d_down=ref.lora_down.weight.grad, d_up=ref.lora_up.weight.grad).items()})
+    torch.save(ops, f"{OUT}/reference_modules_fp32.pt")
+
+    # ---- site order of the extended inject: module path and factor shapes of every site
+    torch.manual_seed(0)
+    u1 = UNet2DConditionModel(UNetConfig.tiny())
+    R.inject_trainable_lora_extended(u1, r=4)
+    out["extended_targets"] = sorted(R.UNET_EXTENDED_TARGET_REPLACE)
+    out["inject_order"] = [[p, list(m.lora_up.weight.shape), list(m.lora_down.weight.shape)]
+                           for p, m in u1.named_modules() if type(m).__name__.startswith("LoraInjected")]
+
+    # ---- small helpers on the tiny UNet
+    torch.manual_seed(0)
+    base = UNet2DConditionModel(UNetConfig.tiny())
+    ours, ref = copy.deepcopy(base), copy.deepcopy(base)
+    rec = {"find_children": [[type(p).__name__, n, list(c.weight.shape)]
+                             for p, n, c in R._find_children(ref, [nn.Linear, nn.Conv2d])]}
+    torch.manual_seed(1)
+    L.inject_trainable_lora(ours, r=4)
+    torch.manual_seed(1)
+    R.inject_trainable_lora(ref, r=4)
+    rec["down"] = [digest(m.lora_down.weight) for m in _sites(ref)]
+    g = torch.Generator().manual_seed(2)
+    for so, sr in zip(_sites(ours), _sites(ref)):
+        so.lora_up.weight.data.normal_(0, 0.02, generator=g)
+        sr.lora_up.weight.data.copy_(so.lora_up.weight.data)
+    rec["ups_down"] = [[digest(u.weight), digest(d.weight)] for u, d in R.extract_lora_ups_down(ref)]
+    R.save_lora_as_json(ref, os.path.join(tmp, "r.json"))
+    with open(os.path.join(tmp, "r.json"), "rb") as fh:
+        rec["json_sha256"] = hashlib.sha256(fh.read()).hexdigest()
+    R.save_lora_weight(ref, os.path.join(tmp, "r.pt"))
+    rec["pt"] = [digest(t) for t in torch.load(os.path.join(tmp, "r.pt"))]
+    emb = {"<tok>": torch.randn(48, generator=g)}
+    xs = os.path.join(tmp, "x.safetensors")
+    L.save_safeloras_with_embeds({"unet": (ours, L.UNET_DEFAULT_TARGET_REPLACE)}, emb, xs)
+    flat = lambda d: {k: [[digest(torch.as_tensor(t)) for t in v[0]], v[1], sorted(v[2])] for k, v in d.items()}
+    rec["load_safeloras"] = flat(R.load_safeloras(xs))
+    rec["load_safeloras_embeds"] = {k: digest(v) for k, v in R.load_safeloras_embeds(xs).items()}
+    both = R.load_safeloras_both(xs)
+    rec["load_safeloras_both"] = [flat(both[0]), {k: digest(v) for k, v in both[1].items()}]
+    rec["ti_lora_path"] = R._ti_lora_path("a/b.c.pt")
+    rec["text_lora_path"] = R._text_lora_path("a/b.c.pt")
+
+    class Tok:
+        def __init__(self, n):
+            self.v = {f"w{i}": i for i in range(n)}
+
+        def add_tokens(self, t):
+            if t in self.v:
+                return 0
+            self.v[t] = len(self.v)
+            return 1
+
+        def convert_tokens_to_ids(self, t):
+            return self.v[t]
+
+        def __len__(self):
+            return len(self.v)
+    torch.manual_seed(3)
+    te_r = build_text_encoder(tiny=True)
+    V = te_r.get_input_embeddings().weight.shape[0]
+    torch.save(emb, os.path.join(tmp, "e.pt"))
+    with warnings.catch_warnings():
+        warnings.simplefilter("ignore")
+        torch.manual_seed(4)
+        R.load_learned_embed_in_clip(os.path.join(tmp, "e.pt"), te_r, Tok(V), token=None, idempotent=True)
+    rec["learned_embed_table"] = digest(te_r.get_input_embeddings().weight)
+    out["small_helpers"] = rec
+    with open(f"{OUT}/reference_live.json", "w") as fh:
+        json.dump(out, fh, indent=0)
+
+
+def gen_formats(R):
+    """tests/test_formats_cpu.py: lora_manager.lora_join, cli_lora_add.add and the to_ckpt_v2 key
+    conversions of the reference, on the seeded LoRA files the tests write with lora_b200."""
+    import tempfile
+    from safetensors import safe_open
+    from lora_b200.host.unet_sd15 import UNet2DConditionModel, UNetConfig
+    from refgold import canon_metadata, digest
+    from test_formats_cpu import _make_lora_file, _read, _vae_keys
+    tmp = tempfile.mkdtemp()
+    out = {}
+    M = _load_ref("lora_manager.py", "lora_manager")
+    p1 = _make_lora_file(os.path.join(tmp, "a.safetensors"), 3, 4, with_tokens=("<z>", "<y>"))
+    p2 = _make_lora_file(os.path.join(tmp, "b.safetensors"), 4, 4)
+    t, meta, ranks, toks = M.lora_join([safe_open(p, framework="pt", device="cpu") for p in (p1, p2)])
+    out["join"] = {"tensors": {k: digest(v) for k, v in t.items()}, "metadata": canon_metadata(meta),
+                   "ranklist": ranks, "token_sizes": toks}
+    _load_ref("lora.py", "lora")
+    _load_ref("to_ckpt_v2.py", "to_ckpt_v2")
+    A = _load_ref("cli_lora_add.py", "cli_lora_add")
+    p1 = _make_lora_file(os.path.join(tmp, "c.safetensors"), 11, 4, with_tokens=("<a>",))
+    p2 = _make_lora_file(os.path.join(tmp, "d.safetensors"), 12, 4, with_tokens=("<b>",))
+    out["add"] = {}
+    for mode in ("lpl", "ljl"):
+        r = os.path.join(tmp, f"r_{mode}.safetensors")
+        A.add(p1, p2, r, 0.7, 0.4, mode=mode)
+        tr, mr = _read(r)
+        out["add"][mode] = {"tensors": {k: digest(v) for k, v in tr.items()}, "metadata": canon_metadata(mr)}
+    C = _load_ref("to_ckpt_v2.py", "to_ckpt_v2")
+    unet_sd = {k: torch.zeros(1) for k in UNet2DConditionModel(UNetConfig.tiny()).state_dict()}
+    out["ckpt_unet_keys"] = list(C.convert_unet_state_dict(dict(unet_sd)))
+    vae_sd = {k: (torch.zeros(4, 4) if ".attentions.0." in k and k.endswith("weight") and "group_norm" not in k
+                  else torch.zeros(4)) for k in _vae_keys()}
+    out["ckpt_vae"] = [[k, list(v.shape)] for k, v in C.convert_vae_state_dict(dict(vae_sd)).items()]
+    with open(f"{OUT}/reference_formats.json", "w") as fh:
+        json.dump(out, fh, indent=0)
+
+
+GENERATORS = {"ops": gen_ops, "ctor_rng": gen_ctor_rng, "inject": gen_inject, "manifest": gen_manifest,
+              "svd": gen_svd, "adamw": lambda R: gen_adamw(), "loss_step": gen_loss_step, "ti": gen_ti,
+              "tuning": gen_tuning, "live": gen_live, "formats": gen_formats}
+
 if __name__ == "__main__":
+    # python scripts/make_golden.py [name ...]   (default: every generator)
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
     R = load_ref_lora()
-    gen_ops(R)
-    gen_ctor_rng(R)
-    gen_inject(R)
-    gen_manifest(R)
-    gen_svd(R)
-    gen_adamw()
-    gen_loss_step(R)
-    gen_ti(R)
-    gen_tuning(R)
+    for name in sys.argv[1:] or GENERATORS:
+        GENERATORS[name](R)
     for fn in sorted(os.listdir(OUT)):
         print(fn, os.path.getsize(f"{OUT}/{fn}"))

@@ -14,7 +14,6 @@ from lora_b200.host.clip import build_text_encoder
 from lora_b200.host.unet_sd15 import UNet2DConditionModel, UNetConfig
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
-REF_LORAS = "/root/reference/example_loras"
 
 
 def _sites(model):
@@ -224,10 +223,12 @@ def test_collapse_add_scale_diag_inspect():
     assert torch.allclose(lin.lora_down.weight.data, 2.0 * torch.ones(4, 16) + 0.5 * down0)
 
 
-def test_fixture_manifest_layout():
+def test_fixture_manifest_layout(tmp_path):
     """The ten fixture files of the reference pin the on-disk layout (SURVEY.md 4). The manifest
     (keys, shapes, dtypes, metadata, what the reference's own parse_safeloras returned) travels
-    with the repo; where the files themselves are mounted, our parser is run on them too."""
+    with the repo; our parser runs on a file of each manifest's layout (its keys, shapes, dtypes and
+    metadata; zero tensors, the parser reads no values)."""
+    from safetensors.torch import save_file
     man = json.load(open(f"{GOLD}/example_loras_manifest.json"))
     assert len(man) == 10
     torch.manual_seed(0)
@@ -246,13 +247,16 @@ def test_fixture_manifest_layout():
             assert keys[f"unet:{i}:down"][0] == [r, s.linear.in_features]
         assert set(json.loads(ent["metadata"]["unet"])) == set(L.UNET_DEFAULT_TARGET_REPLACE)
         assert json.loads(ent["metadata"]["text_encoder"]) == ["CLIPAttention"]
-        if os.path.isdir(REF_LORAS):
-            f = safe_open(f"{REF_LORAS}/{fn}", framework="pt")
-            ours = L.parse_safeloras(f)
-            for name, info in ent["parsed"].items():
-                w, ranks, targets = ours[name]
-                assert len(w) == info["n_weights"] and ranks == info["ranks"] and sorted(targets) == info["targets"]
-            assert sorted(L.parse_safeloras_embeds(f)) == ent["embeds"]
+        path = str(tmp_path / fn)
+        save_file({k: torch.zeros(shape, dtype=getattr(torch, dt)) for k, (shape, dt, _) in keys.items()},
+                  path, metadata=ent["metadata"])
+        f = safe_open(path, framework="pt")
+        ours = L.parse_safeloras(f)
+        assert sorted(ours) == sorted(ent["parsed"])
+        for name, info in ent["parsed"].items():
+            w, ranks, targets = ours[name]
+            assert len(w) == info["n_weights"] and ranks == info["ranks"] and sorted(targets) == info["targets"]
+        assert sorted(L.parse_safeloras_embeds(f)) == ent["embeds"]
 
 
 def test_lr_schedule_restates_diffusers_linear_and_constant():

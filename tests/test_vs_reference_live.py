@@ -1,10 +1,9 @@
-"""Live comparison with the REAL reference module (/root/reference/lora_diffusion/lora.py loaded
-by file path). Runs only where the reference tree is mounted (the build container); on the GPU
-box these are covered by the golden vectors the same module produced."""
+"""Side-by-side comparison with the original lora_diffusion/lora.py on the tiny host models. The
+original's side of every comparison was recorded by running it on the same seeded calls
+(scripts/make_golden.py -> tests/golden/reference_live.json, reference_modules_fp32.pt); tensors
+are compared through content digests (tests/refgold.py), so every equality stays exact."""
 import copy
-import importlib.util
-import json
-import os
+import hashlib
 
 import pytest
 import torch
@@ -15,193 +14,138 @@ import lora_b200 as L
 from lora_b200.host.clip import build_text_encoder
 from lora_b200.host.unet_sd15 import UNet2DConditionModel, UNetConfig
 from oracle.ref_modules import RefLoraSite, ref_inject
-
-REF_FILE = "/root/reference/lora_diffusion/lora.py"
-pytestmark = pytest.mark.skipif(not os.path.exists(REF_FILE), reason="reference tree not mounted")
+from refgold import GOLD, canon_metadata, canon_signature, digest, load
 
 
 @pytest.fixture(scope="module")
-def R():
-    spec = importlib.util.spec_from_file_location("ref_lora_live", REF_FILE)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod
+def G():
+    return load("reference_live.json")
 
 
 def _sites(model):
     return [m for m in model.modules() if type(m).__name__.startswith("LoraInjected")]
 
 
-def _same_signature(a, b, name):
-    import inspect
-    pa, pb = inspect.signature(a).parameters, inspect.signature(b).parameters
-    assert list(pa) == list(pb), name                       # names and order
-    for k in pa:
-        assert pa[k].default == pb[k].default, (name, k)    # defaults (sets compare by value)
-
-
-def test_public_names_cover_the_reference_namespace(R):
-    ref_names = {n for n in dir(R) if not n.startswith("_") and (callable(getattr(R, n)) or n.isupper()
-                 or n in ("safetensors_available",))}
-    skip = {"Callable", "Dict", "List", "Optional", "Set", "Tuple", "Type", "Union", "groupby", "F", "nn",
-            "np", "PIL", "torch", "json", "math", "_find_modules_old"}
-    import inspect
-    ref_names = {n for n in ref_names if n not in skip and not inspect.ismodule(getattr(R, n))}
-    missing = sorted(n for n in ref_names if not hasattr(L, n))
+def test_public_names_cover_the_reference_namespace(G):
+    missing = sorted(n for n in G["namespace"] if not hasattr(L, n))
     assert missing == [], missing
-    for n in ("inject_trainable_lora", "inject_trainable_lora_extended", "monkeypatch_or_replace_lora",
-              "monkeypatch_or_replace_lora_extended", "patch_pipe", "save_all", "tune_lora_scale",
-              "monkeypatch_add_lora", "apply_learned_embed_in_clip", "extract_lora_as_tensor"):
-        _same_signature(getattr(L, n), getattr(R, n), n)
-    _same_signature(L.LoraInjectedLinear.__init__, R.LoraInjectedLinear.__init__, "LoraInjectedLinear")
-    _same_signature(L.LoraInjectedConv2d.__init__, R.LoraInjectedConv2d.__init__, "LoraInjectedConv2d")
+    for name, want in G["signatures"].items():
+        obj = L
+        for part in name.split("."):
+            obj = getattr(obj, part)
+        assert canon_signature(obj) == want, name      # names, order and defaults
 
 
-def test_inject_save_load_equal_reference_on_tiny_models(R, tmp_path):
+def test_inject_save_load_equal_reference_on_tiny_models(G, tmp_path):
+    g0 = G["inject_save_load"]
     torch.manual_seed(0)
     unet = UNet2DConditionModel(UNetConfig.tiny())
     te = build_text_encoder(tiny=True)
-    unet_r, te_r = copy.deepcopy(unet), copy.deepcopy(te)
     torch.manual_seed(1)
     _, n1 = L.inject_trainable_lora_extended(unet, r=4)
     _, t1 = L.inject_trainable_lora(te, target_replace_module={"CLIPAttention"}, r=4)
-    torch.manual_seed(1)
-    _, n2 = R.inject_trainable_lora_extended(unet_r, r=4)
-    _, t2 = R.inject_trainable_lora(te_r, target_replace_module={"CLIPAttention"}, r=4)
-    assert n1 == n2 and t1 == t2
-    ours, refs = _sites(unet) + _sites(te), _sites(unet_r) + _sites(te_r)
-    assert [type(m).__name__ for m in ours] == [type(m).__name__ for m in refs]
-    for a, b in zip(ours, refs):          # same RNG consumption => identical initial factors
-        assert torch.equal(a.lora_down.weight, b.lora_down.weight)
+    assert n1 == g0["unet_names"] and t1 == g0["text_names"]
+    ours = _sites(unet) + _sites(te)
+    assert [type(m).__name__ for m in ours] == g0["kinds"]
+    # same RNG consumption => identical initial factors
+    assert [digest(m.lora_down.weight) for m in ours] == g0["down"]
     g = torch.Generator().manual_seed(2)
-    for a, b in zip(ours, refs):
+    for a in ours:
         a.lora_up.weight.data.normal_(0, 0.05, generator=g)
-        b.lora_up.weight.data.copy_(a.lora_up.weight.data)
-    L.tune_lora_scale(unet, 0.7); R.tune_lora_scale(unet_r, 0.7)
+    L.tune_lora_scale(unet, 0.7)
     L.save_all(unet, te, str(tmp_path / "a.safetensors"), save_ti=False,
                target_replace_module_unet=L.UNET_EXTENDED_TARGET_REPLACE)
-    R.save_all(unet_r, te_r, str(tmp_path / "b.safetensors"), save_ti=False,
-               target_replace_module_unet=R.UNET_EXTENDED_TARGET_REPLACE)
-    fa, fb = safe_open(str(tmp_path / "a.safetensors"), "pt"), safe_open(str(tmp_path / "b.safetensors"), "pt")
-    assert sorted(fa.keys()) == sorted(fb.keys())
-    assert all(torch.equal(fa.get_tensor(k), fb.get_tensor(k)) for k in fa.keys())
-    # cross-loading: the reference patches a model from OUR file and vice versa
+    fa = safe_open(str(tmp_path / "a.safetensors"), "pt")
+    assert sorted(fa.keys()) == sorted(g0["saved"])
+    assert {k: digest(fa.get_tensor(k)) for k in fa.keys()} == g0["saved"]
+    # same keys, tensors and metadata as the reference's file: the reference's loader would read ours
+    # exactly as it read its own, which is what "loaded" recorded
+    assert canon_metadata(fa.metadata()) == g0["saved_metadata"]
+
     class P:
         pass
-    pr, po = P(), P()
+    po = P()
     torch.manual_seed(0)
-    pr.unet, pr.text_encoder = UNet2DConditionModel(UNetConfig.tiny()), build_text_encoder(tiny=True)
-    po.unet, po.text_encoder = copy.deepcopy(pr.unet), copy.deepcopy(pr.text_encoder)
-    R.monkeypatch_or_replace_safeloras(pr, fa)
-    L.monkeypatch_or_replace_safeloras(po, fb)
-    for a, b in zip(_sites(po.unet) + _sites(po.text_encoder), _sites(pr.unet) + _sites(pr.text_encoder)):
-        assert type(a).__name__ == type(b).__name__
-        assert torch.equal(a.lora_up.weight, b.lora_up.weight) and torch.equal(a.lora_down.weight, b.lora_down.weight)
-    L.collapse_lora(po.unet, 0.5); R.collapse_lora(pr.unet, 0.5)
-    for a, b in zip(_sites(po.unet), _sites(pr.unet)):
-        wa = a.linear.weight if hasattr(a, "linear") else a.conv.weight
-        wb = b.linear.weight if hasattr(b, "linear") else b.conv.weight
-        assert torch.equal(wa, wb)
+    po.unet, po.text_encoder = UNet2DConditionModel(UNetConfig.tiny()), build_text_encoder(tiny=True)
+    L.monkeypatch_or_replace_safeloras(po, fa)
+    got = [[type(m).__name__, digest(m.lora_up.weight), digest(m.lora_down.weight)]
+           for m in _sites(po.unet) + _sites(po.text_encoder)]
+    assert got == g0["loaded"]
+    L.collapse_lora(po.unet, 0.5)
+    assert [digest(m.linear.weight if hasattr(m, "linear") else m.conv.weight)
+            for m in _sites(po.unet)] == g0["collapsed"]
 
 
-def test_oracle_modules_equal_reference_modules_fp32(R):
+def test_oracle_modules_equal_reference_modules_fp32():
     """oracle/ref_modules.RefLoraSite vs the reference operator classes, random inputs, fwd+bwd."""
-    torch.manual_seed(3)
-    for conv in (False, True):
-        if conv:
+    cases = torch.load(f"{GOLD}/reference_modules_fp32.pt")
+    assert len(cases) == 2
+    for c in cases:
+        if c["W"].dim() == 4:
             base = nn.Conv2d(8, 12, 3, padding=1)
-            ref = R.LoraInjectedConv2d(8, 12, 3, 1, 1, r=4, dropout_p=0.0, scale=1.3)
-            ref.conv.weight, ref.conv.bias = base.weight, base.bias
-            x = torch.randn(2, 8, 7, 7)
         else:
             base = nn.Linear(24, 40)
-            ref = R.LoraInjectedLinear(24, 40, True, r=4, dropout_p=0.0, scale=1.3)
-            ref.linear.weight, ref.linear.bias = base.weight, base.bias
-            x = torch.randn(3, 5, 24)
-        ref.lora_up.weight.data.normal_(0, 0.1)
+        base.weight.data.copy_(c["W"]); base.bias.data.copy_(c["b"])
         site = RefLoraSite(base, r=4, dropout_p=0.0, scale=1.3)
-        site.down.data.copy_(ref.lora_down.weight.data); site.up.data.copy_(ref.lora_up.weight.data)
-        x1, x2 = x.clone().requires_grad_(True), x.clone().requires_grad_(True)
-        y1, y2 = ref(x1), site(x2)
-        gy = torch.randn_like(y1)
-        y1.backward(gy); y2.backward(gy)
-        assert torch.allclose(y1, y2, atol=1e-5)
-        assert torch.allclose(x1.grad, x2.grad, atol=1e-5)
-        assert torch.allclose(ref.lora_down.weight.grad, site.down.grad, atol=1e-5)
-        assert torch.allclose(ref.lora_up.weight.grad, site.up.grad, atol=1e-5)
+        site.down.data.copy_(c["down"]); site.up.data.copy_(c["up"])
+        x = c["x"].clone().requires_grad_(True)
+        y = site(x)
+        y.backward(c["gy"])
+        assert torch.allclose(c["y"], y, atol=1e-5)
+        assert torch.allclose(c["dX"], x.grad, atol=1e-5)
+        assert torch.allclose(c["d_down"], site.down.grad, atol=1e-5)
+        assert torch.allclose(c["d_up"], site.up.grad, atol=1e-5)
 
 
-def test_oracle_inject_order_equals_reference(R):
+def test_oracle_inject_order_equals_reference(G):
     torch.manual_seed(0)
-    u1 = UNet2DConditionModel(UNetConfig.tiny())
-    u2 = copy.deepcopy(u1)
-    R.inject_trainable_lora_extended(u1, r=4)
-    sites = ref_inject(u2, R.UNET_EXTENDED_TARGET_REPLACE, r=4, extended=True)
-    ref_sites = _sites(u1)
-    assert len(sites) == len(ref_sites)
-    for a, b in zip(sites, ref_sites):
-        assert tuple(a.up.shape) == tuple(b.lora_up.weight.shape)
-        assert tuple(a.down.shape) == tuple(b.lora_down.weight.shape)
-        wb = b.linear.weight if hasattr(b, "linear") else b.conv.weight
-        assert a.weight is not None and torch.equal(a.weight, wb)
+    u2 = UNet2DConditionModel(UNetConfig.tiny())
+    plain = copy.deepcopy(u2)
+    sites = ref_inject(u2, set(G["extended_targets"]), r=4, extended=True)
+    assert len(sites) == len(G["inject_order"])
+    for a, (path, up, down) in zip(sites, G["inject_order"]):
+        assert list(a.up.shape) == up and list(a.down.shape) == down
+        # the reference's site at `path` wraps the layer found there in the un-injected model
+        assert a.weight is not None and torch.equal(a.weight, plain.get_submodule(path).weight)
 
 
-def test_small_helpers_equal_reference(R, tmp_path):
+def test_small_helpers_equal_reference(G, tmp_path):
     """The remaining small public functions, side by side with the reference on the tiny UNet:
     _find_children, extract_lora_ups_down, save_lora_as_json, save_lora_weight (.pt),
     load_safeloras / load_safeloras_embeds / load_safeloras_both, _ti_lora_path,
     load_learned_embed_in_clip."""
-    import filecmp
+    g0 = G["small_helpers"]
     torch.manual_seed(0)
-    base = UNet2DConditionModel(UNetConfig.tiny())
-    ours, ref = copy.deepcopy(base), copy.deepcopy(base)
+    ours = UNet2DConditionModel(UNetConfig.tiny())
     # _find_children: same (parent, name, child) walk on an un-injected model
-    a = [(type(p).__name__, n, tuple(c.weight.shape)) for p, n, c in L._find_children(ours, [nn.Linear, nn.Conv2d])]
-    b = [(type(p).__name__, n, tuple(c.weight.shape)) for p, n, c in R._find_children(ref, [nn.Linear, nn.Conv2d])]
-    assert a == b and len(a) > 20
+    a = [[type(p).__name__, n, list(c.weight.shape)] for p, n, c in L._find_children(ours, [nn.Linear, nn.Conv2d])]
+    assert a == g0["find_children"] and len(a) > 20
     torch.manual_seed(1)
     L.inject_trainable_lora(ours, r=4)
-    torch.manual_seed(1)
-    R.inject_trainable_lora(ref, r=4)
+    assert [digest(s.lora_down.weight) for s in _sites(ours)] == g0["down"]      # ctor RNG parity
     g = torch.Generator().manual_seed(2)
-    for so, sr in zip(_sites(ours), _sites(ref)):
-        assert torch.equal(so.lora_down.weight, sr.lora_down.weight)      # ctor RNG parity
+    for so in _sites(ours):
         so.lora_up.weight.data.normal_(0, 0.02, generator=g)
-        sr.lora_up.weight.data.copy_(so.lora_up.weight.data)
-    eo, er = L.extract_lora_ups_down(ours), R.extract_lora_ups_down(ref)
-    assert len(eo) == len(er) == len(_sites(ours))
-    assert all(torch.equal(x[0].weight, y[0].weight) and torch.equal(x[1].weight, y[1].weight) for x, y in zip(eo, er))
+    eo = L.extract_lora_ups_down(ours)
+    assert len(eo) == len(_sites(ours))
+    assert [[digest(u.weight), digest(d.weight)] for u, d in eo] == g0["ups_down"]
     # json / .pt writers: identical bytes (json) and identical tensors (.pt)
     L.save_lora_as_json(ours, str(tmp_path / "o.json"))
-    R.save_lora_as_json(ref, str(tmp_path / "r.json"))
-    assert filecmp.cmp(tmp_path / "o.json", tmp_path / "r.json", shallow=False)
+    assert hashlib.sha256((tmp_path / "o.json").read_bytes()).hexdigest() == g0["json_sha256"]
     L.save_lora_weight(ours, str(tmp_path / "o.pt"))
-    R.save_lora_weight(ref, str(tmp_path / "r.pt"))
-    wo, wr = torch.load(tmp_path / "o.pt"), torch.load(tmp_path / "r.pt")
-    assert len(wo) == len(wr) and all(torch.equal(x, y) for x, y in zip(wo, wr))
+    assert [digest(t) for t in torch.load(tmp_path / "o.pt")] == g0["pt"]
     # safetensors loaders
     emb = {"<tok>": torch.randn(48, generator=g)}
     L.save_safeloras_with_embeds({"unet": (ours, L.UNET_DEFAULT_TARGET_REPLACE)}, emb, str(tmp_path / "x.safetensors"))
-    for fn in ("load_safeloras", "load_safeloras_embeds", "load_safeloras_both"):
-        go, gr = getattr(L, fn)(str(tmp_path / "x.safetensors")), getattr(R, fn)(str(tmp_path / "x.safetensors"))
-        flat = lambda d: {k: ([torch.as_tensor(t) for t in v[0]], v[1], sorted(v[2])) for k, v in d.items()} \
-            if all(isinstance(v, tuple) for v in d.values()) else d
-        if fn == "load_safeloras_both":
-            go, gr = (flat(go[0]), go[1]), (flat(gr[0]), gr[1])
-            assert go[1].keys() == gr[1].keys() and all(torch.equal(go[1][k], gr[1][k]) for k in gr[1])
-            go, gr = go[0], gr[0]
-        elif fn == "load_safeloras":
-            go, gr = flat(go), flat(gr)
-        else:
-            assert go.keys() == gr.keys() and all(torch.equal(go[k], gr[k]) for k in gr)
-            continue
-        assert go.keys() == gr.keys()
-        for k in gr:
-            assert go[k][1] == gr[k][1] and go[k][2] == gr[k][2]
-            assert all(torch.equal(x, y) for x, y in zip(go[k][0], gr[k][0]))
-    assert L._ti_lora_path("a/b.c.pt") == R._ti_lora_path("a/b.c.pt")
-    assert L._text_lora_path("a/b.c.pt") == R._text_lora_path("a/b.c.pt")
-    # learned-embedding loader on two identical tiny text encoders with a duck tokenizer
+    flat = lambda d: {k: [[digest(torch.as_tensor(t)) for t in v[0]], v[1], sorted(v[2])] for k, v in d.items()}
+    xs = str(tmp_path / "x.safetensors")
+    assert flat(L.load_safeloras(xs)) == g0["load_safeloras"]
+    assert {k: digest(v) for k, v in L.load_safeloras_embeds(xs).items()} == g0["load_safeloras_embeds"]
+    both = L.load_safeloras_both(xs)
+    assert [flat(both[0]), {k: digest(v) for k, v in both[1].items()}] == g0["load_safeloras_both"]
+    assert L._ti_lora_path("a/b.c.pt") == g0["ti_lora_path"]
+    assert L._text_lora_path("a/b.c.pt") == g0["text_lora_path"]
+    # learned-embedding loader on a tiny text encoder with a duck tokenizer
     class Tok:
         def __init__(self, n):
             self.v = {f"w{i}": i for i in range(n)}
@@ -219,7 +163,6 @@ def test_small_helpers_equal_reference(R, tmp_path):
             return len(self.v)
     torch.manual_seed(3)
     te_o = build_text_encoder(tiny=True)
-    te_r = copy.deepcopy(te_o)
     V = te_o.get_input_embeddings().weight.shape[0]
     torch.save(emb, tmp_path / "e.pt")
     import warnings
@@ -227,7 +170,5 @@ def test_small_helpers_equal_reference(R, tmp_path):
         warnings.simplefilter("ignore")
         torch.manual_seed(4)
         L.load_learned_embed_in_clip(str(tmp_path / "e.pt"), te_o, Tok(V), token=None, idempotent=True)
-        torch.manual_seed(4)
-        R.load_learned_embed_in_clip(str(tmp_path / "e.pt"), te_r, Tok(V), token=None, idempotent=True)
-    assert torch.equal(te_o.get_input_embeddings().weight, te_r.get_input_embeddings().weight)
+    assert digest(te_o.get_input_embeddings().weight) == g0["learned_embed_table"]
     assert torch.equal(te_o.get_input_embeddings().weight[V], emb["<tok>"])
